@@ -2,6 +2,7 @@
 """bench.py - BASELINE.json's metric on BASELINE.json's configs, one JSON line on stdout.
 
   python bench.py [--gpus N --steps K --warmup W]           our arm (CUDA kernels through the C ABI)
+  python bench.py --dump-outputs DIR [...]                 ... and write the headline's result as DIR/<name>.npy
   python bench.py --impl reference [...]                     the reference's CPU operators (oracle/_ref)
 
 Workloads (synthetic TPC-H / SSB-shaped columns, defined once as DuckDB SQL and restated with torch ops in
@@ -79,6 +80,27 @@ def traffic_of(traffic, key, rows):
     if not t:
         return None, None
     return int(round(t["dram_bytes_per_row"] * rows)), t.get("source")
+
+
+AGG_RESULT_COLUMNS = ("rf", "ls", "sum_qty", "sum_base_price", "sum_disc_price", "sum_charge", "avg_qty", "avg_price",
+                      "avg_disc", "count_order")
+
+
+def dump_agg_outputs(outdir, res):
+    """The headline aggregate's result as outdir/agg_<column>.npy (float64), rows ordered by the group keys: the
+    device hands the groups back in hash-table order, which may differ between builds.  float64 keeps only the top 53
+    bits of a 128-bit sum, so each sum is also written exactly as agg_<column>_limbs.npy: its four 32-bit limbs in
+    two's complement, least significant first."""
+    os.makedirs(outdir, exist_ok=True)
+    order = np.lexsort((res[1][0], res[0][0]))
+    for name, (vals, _) in zip(AGG_RESULT_COLUMNS, res):
+        vals = vals[order]
+        if vals.dtype == object:
+            words = [int(v) % (1 << 128) for v in vals]
+            limbs = np.array([[(w >> (32 * i)) & 0xFFFFFFFF for i in range(4)] for w in words], dtype=np.float64)
+            np.save(os.path.join(outdir, f"agg_{name}_limbs.npy"), limbs.reshape(len(words), 4))
+            vals = np.array([float(v) for v in vals])
+        np.save(os.path.join(outdir, f"agg_{name}.npy"), vals.astype(np.float64))
 
 
 class ClockSampler:
@@ -295,7 +317,11 @@ def main():
                     help="multi-GPU join plan(s) to measure")
     ap.add_argument("--duckdb-sf", type=float, default=1.0, help="TPC-H scale factor of the e2e_duckdb leg")
     ap.add_argument("--skip", default="", help="comma list of legs to skip: ssb,q3,join,scan,e2e,duckdb,cpu")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the headline aggregate's result of the last timed step "
+                                                          "as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference_arm(args, emit)
         return
@@ -465,6 +491,8 @@ def main():
     cnt_total = int(res[9][0].sum())
     assert cnt_total == n * world, (cnt_total, n * world)
     assert sum(int(x) for x in res[2][0]) == sum_over_ranks(int(q1["qty"].sum().item())), "sum(qty) mismatch"
+    if args.dump_outputs and rank == 0:
+        dump_agg_outputs(args.dump_outputs, res)
 
     def groups_of(res, nkeys):
         return {tuple(int(res[j][0][g]) for j in range(nkeys)): [res[nkeys + a][0][g] for a in range(len(res) - nkeys)]

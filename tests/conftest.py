@@ -1,3 +1,5 @@
+import hashlib
+import json
 import os
 import sys
 
@@ -13,11 +15,25 @@ GOLDEN = os.path.join(ROOT, "tests", "golden")
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box)")
-    config.addinivalue_line("markers", "ref: needs the reference library oracle/_ref/libduckdb_ref.so")
 
 
 def golden(name):
     return np.load(os.path.join(GOLDEN, name), allow_pickle=False)
+
+
+def reference_answers(key):
+    """What the unmodified reference answered for one test's queries (tests/golden/reference_answers.json, written
+    by tests/golden/make_reference_answers.py): small results as rows, large ones as digest() of a canonical form."""
+    with open(os.path.join(GOLDEN, "reference_answers.json")) as f:
+        return json.load(f)[key]
+
+
+def digest(a):
+    """sha256 of an array's dtype, shape and bytes: equal digests mean bit-identical arrays."""
+    a = np.ascontiguousarray(a)
+    h = hashlib.sha256(f"{a.dtype.str}{a.shape}".encode())
+    h.update(a.tobytes())
+    return h.hexdigest()
 
 
 @pytest.fixture(scope="session")
@@ -32,13 +48,3 @@ def ctx():
     yield c
     c.close()
 
-
-@pytest.fixture(scope="session")
-def refcon():
-    from oracle import duckdb_ref as R
-
-    if not R.available():
-        pytest.skip("reference library not built (oracle/_ref/libduckdb_ref.so)")
-    con = R.Connection(threads=4)
-    yield con
-    con.close()

@@ -4,19 +4,18 @@
   enum values a C program sees are the ones duckdb_b200/capi.py declares to ctypes.
 * b200_type / b200_vector_type / b200_expr_op / b200_join_type reuse the numeric values of DuckDB's
   PhysicalType / VectorType / ExpressionType / JoinType (INTEGRATION.md: the shim passes them through without a
-  mapping table).  Checked against the reference headers when /root/reference is present (CPU container only).
+  mapping table).  Checked against the values read from the reference's headers (tests/golden/reference_answers.json).
 """
 import ctypes as C
 import os
-import re
 import subprocess
 
 import pytest
 
+from conftest import reference_answers
 from duckdb_b200 import capi
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
 
 PROBE = r"""
 #include <stddef.h>
@@ -103,32 +102,15 @@ def test_enum_values_match_ctypes_constants(c_view):
             assert capi.DTYPE_OF_TYPE[t].itemsize == size
 
 
-def _reference_enum(path, enum_name):
-    """{NAME: value} of `enum class <enum_name>` in a reference header (C rules: previous + 1 when not explicit)."""
-    text = open(os.path.join(REF, path)).read()
-    m = re.search(r"enum class " + enum_name + r"\b[^{]*\{(.*?)\};", text, re.S)
-    assert m, f"{enum_name} not found in {path}"
-    body = re.sub(r"//[^\n]*", "", m.group(1))
-    values, nxt = {}, 0
-    for item in body.split(","):
-        m = re.match(r"\s*([A-Z_0-9]+)\s*(?:=\s*(\d+))?\s*$", item)
-        if not m:
-            continue
-        nxt = int(m.group(2)) if m.group(2) is not None else nxt
-        values[m.group(1)] = nxt
-        nxt += 1
-    return values
-
-
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "src")), reason="needs the reference tree (CPU container)")
 def test_enum_values_are_duckdbs(c_view):
-    physical = _reference_enum("src/include/duckdb/common/types.hpp", "PhysicalType")
+    duckdb = reference_answers("enums")
+    physical = duckdb["PhysicalType"]
     for ours, theirs in [("B200_BOOL", "BOOL"), ("B200_UINT8", "UINT8"), ("B200_INT8", "INT8"),
                          ("B200_UINT16", "UINT16"), ("B200_INT16", "INT16"), ("B200_UINT32", "UINT32"),
                          ("B200_INT32", "INT32"), ("B200_UINT64", "UINT64"), ("B200_INT64", "INT64"),
                          ("B200_FLOAT", "FLOAT"), ("B200_DOUBLE", "DOUBLE"), ("B200_INT128", "INT128")]:
         assert c_view[("enum", ours)] == physical[theirs], ours
-    expr = _reference_enum("src/include/duckdb/common/enums/expression_type.hpp", "ExpressionType")
+    expr = duckdb["ExpressionType"]
     for ours, theirs in [("B200_EXPR_COLREF", "BOUND_REF"), ("B200_EXPR_CONST", "VALUE_CONSTANT"),
                          ("B200_EXPR_NOT", "OPERATOR_NOT"), ("B200_EXPR_IS_NULL", "OPERATOR_IS_NULL"),
                          ("B200_EXPR_IS_NOT_NULL", "OPERATOR_IS_NOT_NULL"), ("B200_EXPR_EQ", "COMPARE_EQUAL"),
@@ -138,11 +120,11 @@ def test_enum_values_are_duckdbs(c_view):
                          ("B200_EXPR_NOT_DISTINCT", "COMPARE_NOT_DISTINCT_FROM"), ("B200_EXPR_AND", "CONJUNCTION_AND"),
                          ("B200_EXPR_OR", "CONJUNCTION_OR")]:
         assert c_view[("enum", ours)] == expr[theirs], ours
-    join = _reference_enum("src/include/duckdb/common/enums/join_type.hpp", "JoinType")
+    join = duckdb["JoinType"]
     for ours, theirs in [("B200_JOIN_LEFT", "LEFT"), ("B200_JOIN_INNER", "INNER"), ("B200_JOIN_SEMI", "SEMI"),
                          ("B200_JOIN_ANTI", "ANTI"), ("B200_JOIN_MARK", "MARK")]:
         assert c_view[("enum", ours)] == join[theirs], ours
-    vec = _reference_enum("src/include/duckdb/common/enums/vector_type.hpp", "VectorType")
+    vec = duckdb["VectorType"]
     for ours, theirs in [("B200_FLAT_VECTOR", "FLAT_VECTOR"), ("B200_CONSTANT_VECTOR", "CONSTANT_VECTOR"),
                          ("B200_DICTIONARY_VECTOR", "DICTIONARY_VECTOR")]:
         assert c_view[("enum", ours)] == vec[theirs], ours

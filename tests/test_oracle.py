@@ -1,9 +1,9 @@
 """The CPU oracle (oracle/port.py) pinned against the reference's own known-answer vectors, the golden
-fixtures generated from the unmodified reference, and (when present) the live reference library."""
+fixtures generated from the unmodified reference, and the reference's recorded answers on seeded random tables."""
 import numpy as np
 import pytest
 
-from conftest import golden
+from conftest import digest, golden, reference_answers
 from oracle import port as P
 
 
@@ -146,8 +146,11 @@ def test_radix_partition_ids():
     np.testing.assert_array_equal(P.radix_partition_ids(h, 0), [0, 0, 0, 0, 0])
 
 
-@pytest.mark.ref
-def test_port_vs_live_reference_hash_and_groupby(refcon):
+PG_GROUPBY_SQL = ("SELECT k1, k2, sum(x), count(x), count(*), min(x), max(x), avg(x), sum(d), min(d) FROM pg "
+                  "GROUP BY k1, k2")
+
+
+def pg_table():
     rng = np.random.default_rng(7)
     n = 4000
     k1 = rng.integers(-3, 3, size=n).astype(np.int32)
@@ -156,13 +159,17 @@ def test_port_vs_live_reference_hash_and_groupby(refcon):
     x = rng.integers(-10 ** 12, 10 ** 12, size=n).astype(np.int64)
     xv = rng.random(n) > 0.2
     d = rng.standard_normal(n)
-    refcon.execute("DROP TABLE IF EXISTS pg")
-    refcon.load_table("pg", {"k1": (k1, k1v), "k2": k2, "x": (x, xv), "d": d})
-    h = refcon.execute("SELECT hash(k1, k2) FROM pg")[0].values
-    np.testing.assert_array_equal(P.hash_columns([(k1, k1v), (k2, None)]), h)
-    refcon.execute("SET perfect_ht_threshold=0")
-    rows = refcon.fetchall("SELECT k1, k2, sum(x), count(x), count(*), min(x), max(x), avg(x), sum(d), min(d) "
-                           "FROM pg GROUP BY k1, k2")
+    return {"k1": (k1, k1v), "k2": k2, "x": (x, xv), "d": d}
+
+
+def test_port_vs_live_reference_hash_and_groupby():
+    """hash(k1, k2) and a GROUP BY of the port against the reference's answers on the same rows (pg_table)."""
+    t = pg_table()
+    (k1, k1v), k2, (x, xv), d = t["k1"], t["k2"], t["x"], t["d"]
+    n = len(k2)
+    want = reference_answers("port_groupby")
+    assert digest(P.hash_columns([(k1, k1v), (k2, None)])) == want["hash"]
+    rows = [tuple(r) for r in want["rows"]]
     res = P.group_by([(k1, k1v), (k2, None)],
                      [("sum", (x, xv)), ("count", (x, xv)), ("count_star", None), ("min", (x, xv)),
                       ("max", (x, xv)), ("avg", (x, xv)), ("sum", (d, None)), ("min", (d, None))], n)
@@ -175,10 +182,12 @@ def test_port_vs_live_reference_hash_and_groupby(refcon):
         assert got[7] == r[9]
 
 
-@pytest.mark.ref
-def test_port_vs_live_reference_joins(refcon):
-    """every join type of the port against the unmodified reference: NULL keys on both sides, duplicate build
-    keys, composite keys, float keys with NaN / -0.0."""
+JOIN_KEYS_SQL = ["jp.k = jb.k", "jp.k = jb.k AND jp.k2 = jb.k2"]
+FLOAT_JOIN_KEYS = (np.array([0.0, np.nan, 1.5, -0.0, 2.5], dtype=np.float64),
+                   np.array([-0.0, np.nan, 1.5, 7.0, np.nan], dtype=np.float64))
+
+
+def join_tables():
     rng = np.random.default_rng(11)
     nb, npr = 700, 1500
     bk = rng.integers(0, 200, size=nb).astype(np.int64)
@@ -187,40 +196,39 @@ def test_port_vs_live_reference_joins(refcon):
     pk = rng.integers(0, 260, size=npr).astype(np.int64)
     pkv = rng.random(npr) > 0.05
     pk2 = rng.integers(0, 3, size=npr).astype(np.int16)
-    for t in ("jb", "jp"):
-        refcon.execute(f"DROP TABLE IF EXISTS {t}")
-    refcon.load_table("jb", {"k": (bk, bkv), "k2": bk2, "id": np.arange(nb, dtype=np.int32)})
-    refcon.load_table("jp", {"k": (pk, pkv), "k2": pk2, "id": np.arange(npr, dtype=np.int32)})
-    for keys_sql, bkeys, pkeys in [("jp.k = jb.k", [(bk, bkv)], [(pk, pkv)]),
-                                   ("jp.k = jb.k AND jp.k2 = jb.k2", [(bk, bkv), (bk2, None)], [(pk, pkv), (pk2, None)])]:
-        inner = refcon.fetchall(f"SELECT jp.id, jb.id FROM jp JOIN jb ON {keys_sql}")
-        assert sorted(inner) == P.hash_join(bkeys, pkeys, nb, npr, "inner")
-        left = refcon.fetchall(f"SELECT jp.id, jb.id FROM jp LEFT JOIN jb ON {keys_sql}")
-        assert sorted((a, -1 if b is None else b) for a, b in left) == P.hash_join(bkeys, pkeys, nb, npr, "left")
-        semi = refcon.fetchall(f"SELECT jp.id FROM jp SEMI JOIN jb ON {keys_sql}")
-        assert sorted(r[0] for r in semi) == P.hash_join(bkeys, pkeys, nb, npr, "semi")
-        anti = refcon.fetchall(f"SELECT jp.id FROM jp ANTI JOIN jb ON {keys_sql}")
-        assert sorted(r[0] for r in anti) == P.hash_join(bkeys, pkeys, nb, npr, "anti")
-    # MARK join = `k IN (subquery)` in the select list: TRUE / FALSE / NULL per probe row
-    mark = refcon.fetchall("SELECT id, k IN (SELECT k FROM jb) FROM jp ORDER BY id")
+    return ({"k": (bk, bkv), "k2": bk2, "id": np.arange(nb, dtype=np.int32)},
+            {"k": (pk, pkv), "k2": pk2, "id": np.arange(npr, dtype=np.int32)})
+
+
+def join_digest(rows):
+    """canonical form of a join result: sorted (probe id, build id or -1) pairs, or sorted probe ids"""
+    return digest(np.array(sorted(rows), dtype=np.int64))
+
+
+def test_port_vs_live_reference_joins():
+    """every join type of the port against the reference's answers (join_tables): NULL keys on both sides,
+    duplicate build keys, composite keys, float keys with NaN / -0.0."""
+    jb, jp = join_tables()
+    nb, npr = len(jb["id"]), len(jp["id"])
+    bk, bkv = jb["k"]
+    pk, pkv = jp["k"]
+    want = reference_answers("port_joins")
+    for i, (bkeys, pkeys) in enumerate([([(bk, bkv)], [(pk, pkv)]),
+                                        ([(bk, bkv), (jb["k2"], None)], [(pk, pkv), (jp["k2"], None)])]):
+        assert join_digest(P.hash_join(bkeys, pkeys, nb, npr, "inner")) == want[f"inner{i}"]
+        assert join_digest(P.hash_join(bkeys, pkeys, nb, npr, "left")) == want[f"left{i}"]
+        assert join_digest(P.hash_join(bkeys, pkeys, nb, npr, "semi")) == want[f"semi{i}"]
+        assert join_digest(P.hash_join(bkeys, pkeys, nb, npr, "anti")) == want[f"anti{i}"]
+    # MARK join = `k IN (subquery)` in the select list: TRUE / FALSE / NULL (-1) per probe row
     matched, valid = P.hash_join([(bk, bkv)], [(pk, pkv)], nb, npr, "mark")
-    for (_, m), pm, pv in zip(mark, matched, valid):
-        assert (m is None) == (not pv) and (m is None or bool(m) == bool(pm))
+    assert digest(np.where(valid, np.asarray(matched).astype(bool), -1).astype(np.int64)) == want["mark"]
     # float keys: NaN joins NaN, -0.0 joins +0.0 (comparison_operators.cpp:24-40)
-    fb = np.array([0.0, np.nan, 1.5, -0.0, 2.5], dtype=np.float64)
-    fp = np.array([-0.0, np.nan, 1.5, 7.0, np.nan], dtype=np.float64)
-    for t in ("fjb", "fjp"):
-        refcon.execute(f"DROP TABLE IF EXISTS {t}")
-    refcon.load_table("fjb", {"k": fb, "id": np.arange(len(fb), dtype=np.int32)})
-    refcon.load_table("fjp", {"k": fp, "id": np.arange(len(fp), dtype=np.int32)})
-    got = refcon.fetchall("SELECT fjp.id, fjb.id FROM fjp JOIN fjb ON fjp.k = fjb.k")
-    assert sorted(got) == P.hash_join([(fb, None)], [(fp, None)], len(fb), len(fp), "inner")
+    fb, fp = FLOAT_JOIN_KEYS
+    got = P.hash_join([(fb, None)], [(fp, None)], len(fb), len(fp), "inner")
+    assert got == sorted(tuple(r) for r in want["float_inner"])
 
 
-@pytest.mark.ref
-def test_port_vs_live_reference_filters(refcon):
-    """three-valued logic, NULL comparisons, IS [NOT] DISTINCT FROM and the float total order of the port against
-    the reference's WHERE clause, on random data with NULLs / NaN / infinities."""
+def fl_table():
     rng = np.random.default_rng(13)
     n = 3000
     a = rng.integers(-5, 6, size=n).astype(np.int32)
@@ -230,32 +238,41 @@ def test_port_vs_live_reference_filters(refcon):
     f = rng.choice(np.array([np.nan, np.inf, -np.inf, -0.0, 0.0, 1.5, -2.25]), size=n)
     fv = rng.random(n) > 0.1
     g = rng.choice(np.array([np.nan, np.inf, -0.0, 0.0, 1.5, 3.0]), size=n)
-    refcon.execute("DROP TABLE IF EXISTS fl")
-    refcon.load_table("fl", {"id": np.arange(n, dtype=np.int32), "a": (a, av), "b": (b, bv), "f": (f, fv), "g": g})
-    cols = [(a, av), (b, bv), (f, fv), (g, None)]
-    A, B, F, G = ("col", 0), ("col", 1), ("col", 2), ("col", 3)
-    c3 = ("const", 3, np.int32)
-    cases = {
-        "a < b": ("lt", A, B),
-        "a = b OR a > 3": ("or", ("eq", A, B), ("gt", A, c3)),
-        "a <> b AND b <= 3": ("and", ("ne", A, B), ("le", B, c3)),
-        "NOT (a >= b)": ("not", ("ge", A, B)),
-        "a IS NULL OR b IS NOT NULL": ("or", ("isnull", A), ("isnotnull", B)),
-        "a IS DISTINCT FROM b": ("distinct", A, B),
-        "a IS NOT DISTINCT FROM b": ("notdistinct", A, B),
-        "(a < b) IS NULL": ("isnull", ("lt", A, B)),
-        "NOT (a < b AND b < 3) OR a = 3": ("or", ("not", ("and", ("lt", A, B), ("lt", B, c3))), ("eq", A, c3)),
-        "f < g": ("lt", F, G),
-        "f >= g": ("ge", F, G),
-        "f = g": ("eq", F, G),
-        "f <> g": ("ne", F, G),
-        "f IS NOT DISTINCT FROM g": ("notdistinct", F, G),
-        "f > 1.5::DOUBLE": ("gt", F, ("const", 1.5, np.float64)),
-    }
-    for sql, tree in cases.items():
-        exp = sorted(r[0] for r in refcon.fetchall(f"SELECT id FROM fl WHERE {sql}"))
+    return {"id": np.arange(n, dtype=np.int32), "a": (a, av), "b": (b, bv), "f": (f, fv), "g": g}
+
+
+_A, _B, _F, _G = ("col", 0), ("col", 1), ("col", 2), ("col", 3)
+_C3 = ("const", 3, np.int32)
+FL_CASES = {   # WHERE clause -> the port's predicate over (a, b, f, g)
+    "a < b": ("lt", _A, _B),
+    "a = b OR a > 3": ("or", ("eq", _A, _B), ("gt", _A, _C3)),
+    "a <> b AND b <= 3": ("and", ("ne", _A, _B), ("le", _B, _C3)),
+    "NOT (a >= b)": ("not", ("ge", _A, _B)),
+    "a IS NULL OR b IS NOT NULL": ("or", ("isnull", _A), ("isnotnull", _B)),
+    "a IS DISTINCT FROM b": ("distinct", _A, _B),
+    "a IS NOT DISTINCT FROM b": ("notdistinct", _A, _B),
+    "(a < b) IS NULL": ("isnull", ("lt", _A, _B)),
+    "NOT (a < b AND b < 3) OR a = 3": ("or", ("not", ("and", ("lt", _A, _B), ("lt", _B, _C3))), ("eq", _A, _C3)),
+    "f < g": ("lt", _F, _G),
+    "f >= g": ("ge", _F, _G),
+    "f = g": ("eq", _F, _G),
+    "f <> g": ("ne", _F, _G),
+    "f IS NOT DISTINCT FROM g": ("notdistinct", _F, _G),
+    "f > 1.5::DOUBLE": ("gt", _F, ("const", 1.5, np.float64)),
+}
+
+
+def test_port_vs_live_reference_filters():
+    """three-valued logic, NULL comparisons, IS [NOT] DISTINCT FROM and the float total order of the port against
+    the reference's WHERE clause, on random data with NULLs / NaN / infinities (fl_table)."""
+    t = fl_table()
+    n = len(t["id"])
+    cols = [t["a"], t["b"], t["f"], (t["g"], None)]
+    want = reference_answers("port_filters")
+    assert set(want) == set(FL_CASES)
+    for sql, tree in FL_CASES.items():
         sel, _ = P.filter_select(tree, cols, n)
-        assert sel.tolist() == exp, sql
+        assert join_digest(sel.tolist()) == want[sql], sql
 
 
 def test_aggregate_kats_from_reference_tests():
