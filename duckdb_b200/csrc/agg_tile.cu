@@ -18,6 +18,7 @@
 #include "agg_tile.cuh"
 #include <cstring>
 #include <cstdlib>
+#include <type_traits>
 
 struct FastLayout {
 	int n8, n4;
@@ -253,95 +254,213 @@ __global__ void __launch_bounds__(AT_THREADS + 32) agg_fast_kernel(const __grid_
 // ------------------------------------------------------------------ FASTREG
 // FAST specialised for the common TPC-H / SSB shape: <= SLOTS (4 or 8) groups, integer group keys without
 // NULLs, every aggregate is sum / avg / count over NON-NULL 8-byte integer inputs (BIGINT / DECIMAL(<=18)).
-// The per-thread partial sums live in REGISTERS (acc[slot][sum]); a row adds each value to every slot under a
-// predicate (hit[slot]) - no shared-memory traffic for the states, no atomics, and the predicated adds are
-// independent, so the SM issues them back to back.  Values with |x| >= 2^40 (whose per-thread partial could
-// overflow 64 bits) take the global path.
-// acc[j] += x[j] for all j, rows += 1, under one predicate.  Written on the 32-bit halves so that ptxas keeps
-// the low add predicated (3 SASS instructions per 64-bit accumulate instead of add + 2 selects).
-__device__ __forceinline__ void pred_add64(uint64_t &acc, uint64_t x, uint32_t hit) {
-	uint32_t lo = (uint32_t)acc, hi = (uint32_t)(acc >> 32);
-	asm("{\n.reg .pred p;\nsetp.ne.u32 p, %4, 0;\n@p add.cc.u32 %0, %0, %2;\n@p addc.u32 %1, %1, %3;\n}"
-	    : "+r"(lo), "+r"(hi)
-	    : "r"((uint32_t)x), "r"((uint32_t)(x >> 32)), "r"(hit));
-	acc = ((uint64_t)hi << 32) | lo;
+// The per-thread partial sums live in REGISTERS (pa / pb[slot][sum], below); a row adds each value to every slot
+// under that slot's hit predicate - no shared-memory traffic for the states, no atomics, and the adds are
+// independent, so the SM issues them back to back.  Values with |x| >= 2^40 take the global path.
+//
+// A tile is THREADS x FR_ROWS rows, so every consumer thread does the same work.  Thread t owns the row pairs
+// (2t, 2t+1) and (2t + 2 THREADS, 2t + 2 THREADS + 1): one pair of an 8-byte column is one 16-byte shared load,
+// and a warp's loads cover 512 contiguous bytes (no bank conflicts).  A pair whose rows all hit a known slot with
+// small values takes the straight-line path; any other pair, and every row of the ragged last tile, goes through
+// fr_row (directory insert, wide values, overflow to the global table).
+#define FR_ROWS 4
+// dynamic shared memory of one CTA: two CTAs, their static shared memory and the 1 KB per CTA that the
+// system reserves fit the 228 KB of an SM
+#define FR_SMEM_BUDGET (113 * 1024 - 256)
+
+static constexpr int fr_threads(int slots, int nsum) {
+	// registers: SLOTS x NSUM x 2 32-bit accumulators (+ directory + one row pair); two CTAs per SM
+	return slots * nsum <= 20 ? 224 : (slots * nsum <= 32 ? 192 : 160); // + 1 producer warp
+}
+
+// A value x with |x| < 2^40 is accumulated as its two parts x = a * 2^20 + b, a = x >> 20 (signed) and
+// b = x & (2^20 - 1), in 32-bit registers: one predicated 32-bit add per part (2 SASS per slot and sum, no carry
+// chain).  2048 rows per thread keep both part sums inside 32 bits (-2^20 <= a < 2^20, 0 <= b < 2^20); the tile
+// loop folds them into 128-bit per-warp sums in shared memory every FR_FLUSH_TILES tiles.
+#define FR_FLUSH_TILES (2048 / FR_ROWS)
+
+template <int NSUM>
+struct FrVals {
+	uint32_t a[NSUM], b[NSUM];
+	int32_t hmax, hmin; // range of the high words
+};
+
+template <int NSUM>
+__device__ __forceinline__ void fr_split(FrVals<NSUM> &v, int j, uint64_t x) {
+	const uint32_t lo = (uint32_t)x, hi = (uint32_t)(x >> 32);
+	v.a[j] = __funnelshift_r(lo, hi, 20);
+	v.b[j] = lo & 0xfffffu;
+}
+
+// |x| < 2^40 for every value: the high words all lie in [-256, 255]
+__device__ __forceinline__ bool fr_small(int32_t hmax, int32_t hmin) {
+	return hmax < 256 && hmin >= -256;
 }
 
 template <int NSUM>
-__device__ __forceinline__ void pred_accumulate(uint64_t (&acc)[NSUM], uint32_t &rows, const uint64_t (&x)[NSUM],
-                                                uint32_t hit) {
+__device__ __forceinline__ void fr_accumulate(uint32_t (&pa)[NSUM], uint32_t (&pb)[NSUM], uint32_t &rows,
+                                              const FrVals<NSUM> &v, bool hit) {
 #pragma unroll
 	for (int j = 0; j < NSUM; j++) {
-		pred_add64(acc[j], x[j], hit);
+		asm("{\n.reg .pred p;\nsetp.ne.u32 p, %4, 0;\n@p add.u32 %0, %0, %2;\n@p add.u32 %1, %1, %3;\n}"
+		    : "+r"(pa[j]), "+r"(pb[j])
+		    : "r"(v.a[j]), "r"(v.b[j]), "r"((uint32_t)hit));
 	}
-	rows += hit;
+	asm("{\n.reg .pred p;\nsetp.ne.u32 p, %1, 0;\n@p add.u32 %0, %0, 1;\n}" : "+r"(rows) : "r"((uint32_t)hit));
 }
 
-template <int NSUM, int SLOTS, int THREADS, int KW>
-__global__ void __launch_bounds__(THREADS + 32, 2) agg_fastreg_kernel(const __grid_constant__ TileArgs A, RegLayout R) {
-	extern __shared__ __align__(128) unsigned char smem_raw[];
-	__shared__ unsigned long long dir_key[REG_MAX_SLOTS];
-	__shared__ uint64_t gslot[REG_MAX_SLOTS];
-	__shared__ uint64_t bars[2 * AT_MAX_STAGES];
-	const int tid = threadIdx.x;
-	const AggLayout &L = A.L;
-	unsigned char *stages = smem_raw;
-	if (tid < REG_MAX_SLOTS) {
-		dir_key[tid] = 0;
+__device__ __forceinline__ uint32_t lds_u16(uint32_t a) {
+	unsigned short v;
+	asm volatile("ld.shared.u16 %0, [%1];" : "=h"(v) : "r"(a));
+	return v;
+}
+
+__device__ __forceinline__ void lds_v2u32(uint32_t a, uint32_t &x, uint32_t &y) {
+	asm volatile("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(x), "=r"(y) : "r"(a));
+}
+
+__device__ __forceinline__ void lds_v2u64(uint32_t a, uint64_t &x, uint64_t &y) {
+	asm volatile("ld.shared.v2.u64 {%0, %1}, [%2];" : "=l"(x), "=l"(y) : "r"(a));
+}
+
+// Group tags.  KW == 1 (every key column one byte wide, key j in byte j) with NK <= 3 key bytes: the packed key
+// itself, 32 bits, with ~0 (never a key) marking an empty slot.  Otherwise the packed key | 1 << 56 (the
+// directory's format), with 0 marking an empty slot.
+template <int KW, int NK>
+struct FrTag {
+	static constexpr bool narrow = KW == 1 && NK <= 3;
+	using T = typename std::conditional<narrow, uint32_t, unsigned long long>::type;
+	static constexpr T empty = narrow ? (T)~0u : (T)0;
+	__device__ static unsigned long long dir(T t) {
+		return narrow ? (unsigned long long)t | (1ULL << 56) : (unsigned long long)t;
 	}
-	uint64_t acc[SLOTS][NSUM];
-	uint32_t rows[SLOTS];
-	unsigned long long dk[SLOTS];
+	__device__ static T of_packed(uint64_t k) {
+		return narrow ? (T)k : (T)(k | (1ULL << 56));
+	}
+};
+
+// tag of row r of the staged tile
+template <int KW, int NK>
+__device__ __forceinline__ typename FrTag<KW, NK>::T fr_row_tag(const RegLayout &R, const unsigned char *stage, uint32_t r) {
+	uint64_t k = 0;
+	if constexpr (KW == 1) {
+#pragma unroll
+		for (int j = 0; j < NK; j++) {
+			k |= (uint64_t)stage[R.key_smem_off[j] + r] << (8 * j);
+		}
+	} else if constexpr (KW == 4) {
+		k = *(const uint32_t *)(stage + R.key_smem_off[0] + (size_t)r * 4);
+	} else {
+#pragma unroll 1
+		for (int j = 0; j < R.nkeys; j++) {
+			k |= stage_load_uint(stage + R.key_smem_off[j] + r * R.key_width[j], R.key_width[j]) << R.key_shift[j];
+		}
+	}
+	return FrTag<KW, NK>::of_packed(k);
+}
+
+// tags of the row pair (r, r + 1), r even
+template <int KW, int NK>
+__device__ __forceinline__ void fr_pair_tags(const RegLayout &R, const unsigned char *stage, uint32_t sb, uint32_t r,
+                                             typename FrTag<KW, NK>::T &t0, typename FrTag<KW, NK>::T &t1) {
+	if constexpr (KW == 1) {
+		uint32_t a = 0, b = 0;
+#pragma unroll
+		for (int j = 0; j < NK; j++) {
+			uint32_t k = lds_u16(sb + R.key_smem_off[j] + r);
+			a |= (k & 0xffu) << (8 * j);
+			b |= (k >> 8) << (8 * j);
+		}
+		t0 = FrTag<KW, NK>::of_packed(a);
+		t1 = FrTag<KW, NK>::of_packed(b);
+	} else if constexpr (KW == 4) {
+		uint32_t a, b;
+		lds_v2u32(sb + R.key_smem_off[0] + r * 4, a, b);
+		t0 = FrTag<KW, NK>::of_packed(a);
+		t1 = FrTag<KW, NK>::of_packed(b);
+	} else {
+		t0 = fr_row_tag<KW, NK>(R, stage, r);
+		t1 = fr_row_tag<KW, NK>(R, stage, r + 1);
+	}
+}
+
+// 128-bit sum of the warp's per-thread values (lo, hi) into w[0..1] (lane 0 writes; the warp owns w)
+__device__ __forceinline__ void fr_warp_add128(uint64_t *w, uint64_t lo, uint64_t hi) {
+	for (int off = 16; off; off >>= 1) {
+		uint64_t olo = __shfl_xor_sync(0xffffffffu, lo, off);
+		uint64_t ohi = __shfl_xor_sync(0xffffffffu, hi, off);
+		uint64_t v = lo + olo;
+		hi += ohi + (v < lo ? 1 : 0);
+		lo = v;
+	}
+	if ((threadIdx.x & 31) == 0) {
+		uint64_t v = w[0] + lo;
+		w[1] += hi + (v < lo ? 1 : 0);
+		w[0] = v;
+	}
+}
+
+// Fold the consumer thread's part sums into its warp's 128-bit sums wsum[warp][slot][NSUM * 2 + 1] and clear them
+// (warp-collective).
+template <int NSUM, int SLOTS>
+__device__ __forceinline__ void fr_flush(uint64_t *wsum, uint32_t (&pa)[SLOTS][NSUM], uint32_t (&pb)[SLOTS][NSUM]) {
+	uint64_t *w = wsum + (threadIdx.x >> 5) * SLOTS * (NSUM * 2 + 1);
 #pragma unroll
 	for (int s = 0; s < SLOTS; s++) {
-		rows[s] = 0;
-		dk[s] = 0;
 #pragma unroll
 		for (int j = 0; j < NSUM; j++) {
-			acc[s][j] = 0;
+			const int64_t v = (int64_t)(int32_t)pa[s][j] * (1LL << 20) + pb[s][j];
+			fr_warp_add128(w + s * (NSUM * 2 + 1) + 2 * j, (uint64_t)v, v < 0 ? ~0ULL : 0ULL);
+			pa[s][j] = 0;
+			pb[s][j] = 0;
 		}
 	}
-	unsigned long long missed = 0;
+}
 
-	tile_loop(A, stages, bars, THREADS, [&](const unsigned char *stage, uint32_t r, uint64_t row) {
-		// packed key: integer keys without NULLs -> the NULL byte is 0, fields are zero-extended loads
-		unsigned long long tagged = 1ULL << 56;
-		if constexpr (KW == 1) {
-			// every key column is one byte wide (e.g. Q1's two UTINYINT flags): key j sits in byte j
+// The consumer side of agg_fastreg_kernel for one key shape (NK key columns when KW == 1).
+template <int NSUM, int SLOTS, int THREADS, int KW, int NK>
+__device__ __forceinline__ void fr_consume(const TileArgs &A, const RegLayout &R, unsigned char *stages, uint64_t *bars,
+                                           unsigned long long *dir_key, uint64_t *wsum, uint32_t (&rows)[SLOTS],
+                                           unsigned long long &missed) {
+	using Tag = typename FrTag<KW, NK>::T;
+	const uint32_t tid = threadIdx.x;
+	Tag dk[SLOTS];
+	uint32_t pa[SLOTS][NSUM], pb[SLOTS][NSUM];
 #pragma unroll
-			for (int j = 0; j < 4; j++) {
-				if (j < R.nkeys) {
-					tagged |= (unsigned long long)stage[R.key_smem_off[j] + r] << (8 * j);
-				}
-			}
-		} else if constexpr (KW == 4) {
-			tagged |= *(const uint32_t *)(stage + R.key_smem_off[0] + (size_t)r * 4); // one 4-byte key
-		} else {
-#pragma unroll 1
-			for (int j = 0; j < R.nkeys; j++) {
-				tagged |= stage_load_uint(stage + R.key_smem_off[j] + r * R.key_width[j], R.key_width[j])
-				          << R.key_shift[j];
-			}
-		}
-		uint32_t hit[SLOTS];
-		uint32_t any = 0;
-#pragma unroll
-		for (int s = 0; s < SLOTS; s++) {
-			hit[s] = dk[s] == tagged ? 1u : 0u;
-			any |= hit[s];
-		}
-		uint64_t x[NSUM];
-		uint64_t big = 0;
+	for (int s = 0; s < SLOTS; s++) {
+		dk[s] = FrTag<KW, NK>::empty;
 #pragma unroll
 		for (int j = 0; j < NSUM; j++) {
-			x[j] = *(const uint64_t *)(stage + R.sum_smem_off[j] + (size_t)r * 8);
-			big |= (x[j] + (1ULL << 40)) >> 41;
+			pa[s][j] = 0;
+			pb[s][j] = 0;
 		}
-		if (!any || big) {
-			// slow path: first time this thread sees the key (look it up / insert it in the CTA's directory),
-			// or a value too large for the 64-bit private partials
-			uint64_t kw[KEY_WORDS_MAX] = {tagged & ~(0xffULL << 56), 0, 0, 0};
-			int slot = -1;
+	}
+	uint32_t tiles = 0; // since the last flush
+
+	// one row on its own: first sight of a key (directory insert), wide values, more than SLOTS groups
+	auto fr_row = [&](const unsigned char *stage, uint32_t r, uint64_t row) {
+		const Tag tag = fr_row_tag<KW, NK>(R, stage, r);
+		FrVals<NSUM> v;
+		v.hmax = INT32_MIN;
+		v.hmin = INT32_MAX;
+#pragma unroll
+		for (int j = 0; j < NSUM; j++) {
+			const uint64_t x = *(const uint64_t *)(stage + R.sum_smem_off[j] + (size_t)r * 8);
+			fr_split(v, j, x);
+			v.hmax = max(v.hmax, (int32_t)(x >> 32));
+			v.hmin = min(v.hmin, (int32_t)(x >> 32));
+		}
+		const bool big = !fr_small(v.hmax, v.hmin);
+		int slot = -1;
+#pragma unroll
+		for (int s = 0; s < SLOTS; s++) {
+			if (dk[s] == tag) {
+				slot = s;
+			}
+		}
+		if (slot < 0 || big) {
+			const unsigned long long tagged = FrTag<KW, NK>::dir(tag);
+			slot = -1;
 			if (!big) {
 				for (int s = 0; s < SLOTS; s++) {
 					unsigned long long old = atomicCAS(&dir_key[s], 0ULL, tagged);
@@ -355,54 +474,152 @@ __global__ void __launch_bounds__(THREADS + 32, 2) agg_fastreg_kernel(const __gr
 				if (!big) {
 					missed++;
 				}
+				uint64_t kw[KEY_WORDS_MAX] = {tagged & ~(0xffULL << 56), 0, 0, 0};
 				row_to_global(A, stage, r, row, kw);
 				return;
 			}
 #pragma unroll
 			for (int s = 0; s < SLOTS; s++) {
 				if (s == slot) {
-					dk[s] = tagged;
-					hit[s] = 1;
+					dk[s] = tag;
 				}
 			}
 		}
 #pragma unroll
 		for (int s = 0; s < SLOTS; s++) {
-			pred_accumulate<NSUM>(acc[s], rows[s], x, hit[s]);
+			fr_accumulate<NSUM>(pa[s], pb[s], rows[s], v, s == slot);
+		}
+	};
+
+	tp_tile_loop(A.tc, A.stages, stages, bars, A.row_begin, A.row_end, THREADS,
+	             [&](const unsigned char *stage, uint64_t row0, uint32_t rows_in_tile) {
+		// bit i: the thread's row i (pair i / 2, row i % 2 of the pair) goes through fr_row
+		uint32_t slow = 0;
+		if (rows_in_tile == THREADS * FR_ROWS) {
+			const uint32_t sb = tp_smem_addr(stage);
+#pragma unroll
+			for (int p = 0; p < FR_ROWS / 2; p++) {
+				const uint32_t r = 2 * tid + p * 2 * THREADS;
+				Tag t0, t1;
+				fr_pair_tags<KW, NK>(R, stage, sb, r, t0, t1);
+				FrVals<NSUM> v0, v1;
+				int32_t hmax = INT32_MIN, hmin = INT32_MAX;
+#pragma unroll
+				for (int j = 0; j < NSUM; j++) {
+					uint64_t x0, x1;
+					lds_v2u64(sb + R.sum_smem_off[j] + r * 8, x0, x1);
+					fr_split(v0, j, x0);
+					fr_split(v1, j, x1);
+					hmax = __vimax3_s32(hmax, (int32_t)(x0 >> 32), (int32_t)(x1 >> 32));
+					hmin = __vimin3_s32(hmin, (int32_t)(x0 >> 32), (int32_t)(x1 >> 32));
+				}
+				bool h0[SLOTS], h1[SLOTS];
+				bool any0 = false, any1 = false;
+#pragma unroll
+				for (int s = 0; s < SLOTS; s++) {
+					h0[s] = dk[s] == t0;
+					h1[s] = dk[s] == t1;
+					any0 |= h0[s];
+					any1 |= h1[s];
+				}
+				if (any0 && any1 && fr_small(hmax, hmin)) {
+#pragma unroll
+					for (int s = 0; s < SLOTS; s++) {
+						fr_accumulate<NSUM>(pa[s], pb[s], rows[s], v0, h0[s]);
+						fr_accumulate<NSUM>(pa[s], pb[s], rows[s], v1, h1[s]);
+					}
+				} else {
+					slow |= 3u << (2 * p);
+				}
+			}
+		} else {
+#pragma unroll
+			for (int i = 0; i < FR_ROWS; i++) {
+				if (2 * tid + (i >> 1) * 2 * THREADS + (i & 1) < rows_in_tile) {
+					slow |= 1u << i;
+				}
+			}
+		}
+		while (slow) {
+			const int i = __ffs(slow) - 1;
+			slow &= slow - 1;
+			const uint32_t r = 2 * tid + (i >> 1) * 2 * THREADS + (i & 1);
+			fr_row(stage, r, row0 + r);
+		}
+		if (++tiles == FR_FLUSH_TILES) {
+			fr_flush<NSUM, SLOTS>(wsum, pa, pb);
+			tiles = 0;
 		}
 	});
+	if (tid < THREADS) {
+		fr_flush<NSUM, SLOTS>(wsum, pa, pb);
+	}
+}
+
+// dynamic shared memory of a launch: the stage ring, then the per-warp sums
+static constexpr size_t fr_wsum_bytes(int slots, int nsum) {
+	return (size_t)(fr_threads(slots, nsum) / 32) * slots * (nsum * 2 + 1) * 8;
+}
+
+template <int NSUM, int SLOTS, int THREADS, int KW>
+__global__ void __launch_bounds__(THREADS + 32, 2) agg_fastreg_kernel(const __grid_constant__ TileArgs A, RegLayout R) {
+	extern __shared__ __align__(128) unsigned char smem_raw[];
+	__shared__ unsigned long long dir_key[REG_MAX_SLOTS];
+	__shared__ uint64_t gslot[REG_MAX_SLOTS];
+	__shared__ uint64_t bars[2 * AT_MAX_STAGES];
+	constexpr int per_slot = NSUM * 2 + 1;
+	constexpr int nwarps = THREADS / 32;
+	const int tid = threadIdx.x;
+	const AggLayout &L = A.L;
+	unsigned char *stages = smem_raw;
+	uint64_t *wsum = (uint64_t *)(smem_raw + (size_t)A.stages * A.tc.stage_bytes); // [warp][slot][per_slot]
+	if (tid < REG_MAX_SLOTS) {
+		dir_key[tid] = 0;
+	}
+	for (int i = tid; i < nwarps * SLOTS * per_slot; i += blockDim.x) {
+		wsum[i] = 0;
+	}
+	uint32_t rows[SLOTS];
+#pragma unroll
+	for (int s = 0; s < SLOTS; s++) {
+		rows[s] = 0;
+	}
+	unsigned long long missed = 0;
+
+	// (tp_tile_loop synchronises the CTA before its first tile and after its last)
+	if constexpr (KW == 1) {
+		// the number of one-byte key columns is a compile-time value of the row loop
+		switch (R.nkeys) {
+		case 1:
+			fr_consume<NSUM, SLOTS, THREADS, KW, 1>(A, R, stages, bars, dir_key, wsum, rows, missed);
+			break;
+		case 2:
+			fr_consume<NSUM, SLOTS, THREADS, KW, 2>(A, R, stages, bars, dir_key, wsum, rows, missed);
+			break;
+		case 3:
+			fr_consume<NSUM, SLOTS, THREADS, KW, 3>(A, R, stages, bars, dir_key, wsum, rows, missed);
+			break;
+		default:
+			fr_consume<NSUM, SLOTS, THREADS, KW, 4>(A, R, stages, bars, dir_key, wsum, rows, missed);
+			break;
+		}
+	} else {
+		fr_consume<NSUM, SLOTS, THREADS, KW, 0>(A, R, stages, bars, dir_key, wsum, rows, missed);
+	}
 
 	if (missed) {
 		atomicAdd(&A.counters[1], missed);
 	}
-	__syncthreads();
-	// reduce: warp shuffle (128-bit), then across warps through shared memory (the stage buffers are free now)
-	const int lane = tid & 31, warp = tid >> 5, nwarps = THREADS / 32;
-	uint64_t *red = (uint64_t *)stages; // [warp][slot][NSUM*2 + 1]  (the producer warp writes zeros, never read)
-	const int per_slot = NSUM * 2 + 1;
+	const int lane = tid & 31, warp = tid >> 5;
+	if (tid < THREADS) {
 #pragma unroll
-	for (int s = 0; s < SLOTS; s++) {
-		unsigned long long rr = rows[s];
-		for (int off = 16; off; off >>= 1) {
-			rr += __shfl_xor_sync(0xffffffffu, rr, off);
-		}
-		if (lane == 0) {
-			red[(warp * SLOTS + s) * per_slot + NSUM * 2] = rr;
-		}
-#pragma unroll
-		for (int j = 0; j < NSUM; j++) {
-			uint64_t lo = acc[s][j];
-			uint64_t hi = (int64_t)lo < 0 ? ~0ULL : 0ULL; // partials are signed 64-bit values (|.| < 2^62)
+		for (int s = 0; s < SLOTS; s++) {
+			unsigned long long rr = rows[s];
 			for (int off = 16; off; off >>= 1) {
-				uint64_t olo = __shfl_xor_sync(0xffffffffu, lo, off);
-				uint64_t ohi = __shfl_xor_sync(0xffffffffu, hi, off);
-				uint64_t v = lo + olo;
-				hi += ohi + (v < lo ? 1 : 0);
-				lo = v;
+				rr += __shfl_xor_sync(0xffffffffu, rr, off);
 			}
 			if (lane == 0) {
-				red[(warp * SLOTS + s) * per_slot + 2 * j] = lo;
-				red[(warp * SLOTS + s) * per_slot + 2 * j + 1] = hi;
+				wsum[(warp * SLOTS + s) * per_slot + NSUM * 2] = rr;
 			}
 		}
 	}
@@ -410,7 +627,7 @@ __global__ void __launch_bounds__(THREADS + 32, 2) agg_fastreg_kernel(const __gr
 	if (tid < SLOTS) {
 		unsigned long long rr = 0;
 		for (int w = 0; w < nwarps; w++) {
-			rr += red[(w * SLOTS + tid) * per_slot + NSUM * 2];
+			rr += wsum[(w * SLOTS + tid) * per_slot + NSUM * 2];
 		}
 		uint64_t gs = SLOT_DEFER;
 		if (dir_key[tid] != 0ULL && rr) {
@@ -426,8 +643,8 @@ __global__ void __launch_bounds__(THREADS + 32, 2) agg_fastreg_kernel(const __gr
 		if (gslot[s] != SLOT_DEFER) {
 			uint64_t lo = 0, hi = 0;
 			for (int w = 0; w < nwarps; w++) {
-				uint64_t olo = red[(w * SLOTS + s) * per_slot + 2 * j];
-				uint64_t ohi = red[(w * SLOTS + s) * per_slot + 2 * j + 1];
+				uint64_t olo = wsum[(w * SLOTS + s) * per_slot + 2 * j];
+				uint64_t ohi = wsum[(w * SLOTS + s) * per_slot + 2 * j + 1];
 				uint64_t v = lo + olo;
 				hi += ohi + (v < lo ? 1 : 0);
 				lo = v;
@@ -440,15 +657,14 @@ __global__ void __launch_bounds__(THREADS + 32, 2) agg_fastreg_kernel(const __gr
 
 template <int NSUM, int SLOTS, int KW>
 static int launch_fastreg(b200_ctx *ctx, const TileArgs &A, const RegLayout &R, uint64_t ntiles) {
-	// registers: SLOTS x NSUM 64-bit accumulators (+ directory + temporaries); two CTAs per SM
-	constexpr int THREADS = (SLOTS * NSUM <= 20) ? 224 : (SLOTS * NSUM <= 32 ? 192 : 160); // + 1 producer warp
+	constexpr int THREADS = fr_threads(SLOTS, NSUM);
 	static bool attr_set = false;
 	if (!attr_set) {
 		CUDA_TRY(cudaFuncSetAttribute(agg_fastreg_kernel<NSUM, SLOTS, THREADS, KW>,
-		                              cudaFuncAttributeMaxDynamicSharedMemorySize, 110 * 1024));
+		                              cudaFuncAttributeMaxDynamicSharedMemorySize, FR_SMEM_BUDGET));
 		attr_set = true;
 	}
-	size_t smem = (size_t)A.stages * A.tc.stage_bytes;
+	size_t smem = (size_t)A.stages * A.tc.stage_bytes + fr_wsum_bytes(SLOTS, NSUM);
 	uint64_t max_grid = (uint64_t)ctx->sm_count * 2;
 	uint64_t grid = ntiles < max_grid ? ntiles : max_grid;
 	agg_fastreg_kernel<NSUM, SLOTS, THREADS, KW><<<(unsigned)grid, THREADS + 32, smem, ctx->stream>>>(A, R);
@@ -1008,7 +1224,6 @@ int b200_agg_tile_sink(b200_ctx *ctx, int mode, int slots_hint, const AggLayout 
 	tile_cols_finish(&A.tc, AT_TILE);
 	uint64_t n = row_end - row_begin;
 	uint64_t ntiles = (n + AT_TILE - 1) / AT_TILE;
-	const char *tile_env = getenv("B200_AGG_TILE"); // experiment knob for the register fast path: rows per tile
 	static bool attr_set = false;
 	if (!attr_set) {
 		CUDA_TRY(cudaFuncSetAttribute(agg_fast_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, AT_SMEM_BUDGET));
@@ -1033,6 +1248,7 @@ int b200_agg_tile_sink(b200_ctx *ctx, int mode, int slots_hint, const AggLayout 
 		RegLayout R;
 		memset(&R, 0, sizeof(R));
 		bool reg_ok = L.key_bytes <= 7;
+		size_t fr_extra = 0;
 		R.nkeys = L.nkeys;
 		for (int j = 0; j < L.nkeys && reg_ok; j++) {
 			reg_ok = b200_type_is_integer(L.key_type[j]) && !keys.c[j].validity;
@@ -1052,12 +1268,15 @@ int b200_agg_tile_sink(b200_ctx *ctx, int mode, int slots_hint, const AggLayout 
 			}
 		}
 		if (reg_ok && R.nsum >= 1) {
-			// two CTAs per SM: deeper ring of smaller tiles (3 x 512 rows) when it fits, else 2 x 1024
-			uint32_t rows = tile_env && atoi(tile_env) >= 128 ? (uint32_t)atoi(tile_env) / 128 * 128 : 1024;
+			// tiles of FR_ROWS rows per consumer thread; as many stages (up to 3) as fit two CTAs per SM.  Q1
+			// (42 B/row, 896-row tiles): 3 x 37.6 KB, so two tiles per CTA are in flight while it works on a third.
+			const int slots = slots_hint <= 4 ? 4 : 8;
+			uint32_t rows = (uint32_t)fr_threads(slots, R.nsum) * FR_ROWS;
 			tile_cols_finish(&A.tc, rows);
-			A.stages = 3; // measured on B200: 2 x 1024-row stages beat 3 x 512 (per-tile issue cost), see profiles/
-			if ((size_t)A.stages * A.tc.stage_bytes > 108 * 1024) {
-				A.stages = 2;
+			fr_extra = fr_wsum_bytes(slots, R.nsum);
+			A.stages = AT_MAX_STAGES;
+			while (A.stages > 2 && (size_t)A.stages * A.tc.stage_bytes + fr_extra > FR_SMEM_BUDGET) {
+				A.stages--;
 			}
 			ntiles = (n + rows - 1) / rows;
 			for (int j = 0; j < L.nkeys; j++) {
@@ -1067,7 +1286,7 @@ int b200_agg_tile_sink(b200_ctx *ctx, int mode, int slots_hint, const AggLayout 
 				R.sum_smem_off[j] = A.tc.c[A.sm.in_data[R.in_of_sum[j]]].smem_off;
 			}
 		}
-		if (reg_ok && R.nsum >= 1 && (size_t)A.stages * A.tc.stage_bytes <= 108 * 1024) {
+		if (reg_ok && R.nsum >= 1 && (size_t)A.stages * A.tc.stage_bytes + fr_extra <= FR_SMEM_BUDGET) {
 			// first try 4 slots (TPC-H Q1 has 4 groups); the caller escalates to 8 slots, then MID, then GLOBAL
 			int rc = slots_hint <= 4 ? dispatch_fastreg<4>(ctx, A, R, ntiles) : dispatch_fastreg<8>(ctx, A, R, ntiles);
 			ctx->launches++;

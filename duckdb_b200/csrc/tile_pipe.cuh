@@ -181,7 +181,8 @@ __device__ __forceinline__ void tp_consumer_sync(int NC) {
 // (blockDim.x == NC + 32).  The producer's lane 0 walks the CTA's tiles (blockIdx.x, blockIdx.x + gridDim.x, ...)
 // of rows [row_begin, row_end), waits for empty[s] and issues the TMA copies that complete on full[s]; the
 // consumers call body(stage_ptr, row0, rows_in_tile) once per tile.  Inside body use tp_consumer_sync(NC), never
-// __syncthreads().  bars: 2*S mbarriers in shared memory.  row_begin must be a multiple of tc.tile_rows.
+// __syncthreads().  bars: 2*S mbarriers in shared memory.  row_begin must be a multiple of 128 rows (as tc.tile_rows
+// is), so that every column's tile - bit-packed ones included - starts 16-byte aligned.
 template <class BODY>
 __device__ __forceinline__ void tp_tile_loop(const TileCols &tc, int S, unsigned char *stages, uint64_t *bars,
                                              uint64_t row_begin, uint64_t row_end, int NC, BODY body) {
@@ -198,33 +199,38 @@ __device__ __forceinline__ void tp_tile_loop(const TileCols &tc, int S, unsigned
 		tp_fence_mbar_init();
 	}
 	__syncthreads();
+	// the k-th tile of the CTA uses stage k mod S in round k / S; both are kept as counters (S is a run-time value
+	// and a 64-bit `k % S` / `k / S` is a call into the division routine)
+	int s = 0;
+	uint32_t parity = 0; // (k / S) & 1
 	if ((int)threadIdx.x >= NC) {
 		if ((threadIdx.x & 31) == 0) {
-			for (uint64_t k = 0;; k++) {
-				uint64_t t = blockIdx.x + k * gridDim.x;
-				if (t >= nfull) {
-					break;
-				}
-				int s = (int)(k % S);
-				uint64_t use = k / S;
-				if (use >= 1) {
-					tp_wait(&empty[s], (uint32_t)((use - 1) & 1));
+			bool refill = false; // k >= S: wait until the consumers are done with the stage's previous tile
+			for (uint64_t t = blockIdx.x; t < nfull; t += gridDim.x) {
+				if (refill) {
+					tp_wait(&empty[s], parity ^ 1u);
 				}
 				tp_issue_full(tc, stages + (size_t)s * tc.stage_bytes, &full[s], row_begin + t * TILE);
+				if (++s == S) {
+					s = 0;
+					parity ^= 1u;
+					refill = true;
+				}
 			}
 		}
 	} else {
-		for (uint64_t k = 0;; k++) {
-			uint64_t t = blockIdx.x + k * gridDim.x;
-			if (t >= ntiles) {
-				break;
-			}
-			int s = (int)(k % S);
+		for (uint64_t t = blockIdx.x; t < ntiles; t += gridDim.x) {
 			unsigned char *stage = stages + (size_t)s * tc.stage_bytes;
 			uint32_t rows_in_tile = TILE;
 			uint64_t row0 = row_begin + t * TILE;
+			const int s_now = s;
+			const uint32_t parity_now = parity;
+			if (++s == S) {
+				s = 0;
+				parity ^= 1u;
+			}
 			if (t < nfull) {
-				tp_wait(&full[s], (uint32_t)((k / S) & 1));
+				tp_wait(&full[s_now], parity_now);
 			} else {
 				// ragged last tile: plain cooperative copy by the consumers
 				tp_consumer_sync(NC);
@@ -243,7 +249,7 @@ __device__ __forceinline__ void tp_tile_loop(const TileCols &tc, int S, unsigned
 			body(stage, row0, rows_in_tile);
 			__syncwarp();
 			if ((threadIdx.x & 31) == 0) {
-				tp_arrive(&empty[s]);
+				tp_arrive(&empty[s_now]);
 			}
 		}
 	}
